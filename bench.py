@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py — the contract benchmark of the batched TinyMPC solve path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -52,6 +52,9 @@ KERNEL_NAMES = {1: "tpi", 2: "gpi", 4: "gps"}
 # `config` is the same dict in both arms (the driver compares them); arm-specific details go to `plan` / `arm`
 CONFIG = {"workload": WORKLOAD, "instances_per_gpu": B_PER_GPU,
           "l2": "GPU arm: flushed (256 MiB write) between timed steps; CPU arm: every step re-solves the sample from cold state"}
+# --dump-outputs: instances written per config; with every config dumped the files stay below 64 MB in all
+DUMP_INSTANCES = 1024
+DUMP_KEYS = ("sol_x", "sol_u", "iter", "solved", "residuals")
 
 
 def parse():
@@ -66,7 +69,13 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the `configs` block (C3/C4/C5)")
     ap.add_argument("--extra-steps", type=int, default=5)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed solve of each config returned as DIR/<config>_<name>.npy "
+                         f"(float32/float64; at most {DUMP_INSTANCES} instances per config, a fixed seeded sample of larger batches)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.extra_steps < 1:
+        ap.error("--steps and --extra-steps must be >= 1")
+    return args
 
 
 # ---------------------------------------------------------------------------------------------------------
@@ -457,6 +466,22 @@ def plan_of(st):
             "tmem_cols_per_cta": st["tmem_cols_per_cta"], "instances_per_cta": st["instances_per_cta"]}
 
 
+def dump_outputs(dirname, name, out):
+    """Writes the arrays a caller of the timed path receives (`out` of the last timed solve) as float32/float64 .npy files,
+    restricted to a fixed seeded sample of DUMP_INSTANCES instances when the batch is larger, so that two builds run with the
+    same arguments can be compared output for output."""
+    import torch
+
+    B = int(out["iter"].shape[0])
+    idx = np.arange(B) if B <= DUMP_INSTANCES else np.sort(np.random.default_rng(0).choice(B, DUMP_INSTANCES, replace=False))
+    os.makedirs(dirname, exist_ok=True)
+    for key in DUMP_KEYS:
+        a = out[key].index_select(0, torch.as_tensor(idx, device=out[key].device)).cpu().numpy()
+        if a.dtype not in (np.float32, np.float64):
+            a = a.astype(np.float64)  # iter, solved: int32, exact in float64
+        np.save(os.path.join(dirname, f"{name}_{key}.npy"), a)
+
+
 def main():
     args = parse()
     rank = int(os.environ.get("RANK", "0"))
@@ -503,6 +528,8 @@ def main():
     time.sleep(0.25)
     t_wall0 = time.perf_counter()
     batch, out, step_ms = g.device_arm(solver, case, K, W)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, "C2", out)
     total_ms = float(sum(step_ms))
     st = solver.stats()
     iters_step = int(out["iter"].sum().item())
@@ -542,6 +569,8 @@ def main():
             p = setup_problem(c["spec"], c["dtype"])
             s = BatchedTinySolver(p, c["spec"].settings, device=local, mode=mode, kernel=abi.KERNEL_AUTO)
             b_, o_, ms_ = g.device_arm(s, c, Kx, W)
+            if args.dump_outputs and rank == 0:
+                dump_outputs(args.dump_outputs, name, o_)
             sx = s.stats()
             it = o_["iter"]
             iters_x, solved_x = int(it.sum().item()), int(o_["solved"].sum().item())

@@ -2,6 +2,7 @@
 workloads) and a closed-loop runner that feeds warm-start state back the way the reference's examples do."""
 from __future__ import annotations
 
+import hashlib
 import os
 
 import numpy as np
@@ -10,6 +11,9 @@ from tinympc_b200 import abi, workloads as wl
 from tinympc_b200.problem import MPCProblem, copy_settings
 
 GOLDEN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+# further outputs of the unmodified reference (tests/golden/make_golden.py), kept apart from the closed-loop fixtures above
+REF_DIR = os.path.join(GOLDEN_DIR, "reference")
+CACHE_FIELDS = ("Q", "R", "Kinf", "Pinf", "Quu_inv", "AmBKt", "APf", "BPf")
 BOX_STATE = ["x", "u", "v", "z", "vnew", "znew", "g", "y"]
 SOC_STATE = BOX_STATE + ["vcnew", "zcnew", "gc", "yc"]
 LIN_STATE = BOX_STATE + ["vlnew", "zlnew", "gl", "yl"]
@@ -27,6 +31,58 @@ def problem_from_spec(spec: wl.ModelSpec, dtype, setup) -> MPCProblem:
     """setup(nx,nu,N,rho,A,B,f,Qdiag,Rdiag,dtype=..., **constraints) -> MPCProblem (oracle.ref_setup / port_setup)."""
     return setup(spec.nx, spec.nu, spec.N, spec.rho, spec.A, spec.B, spec.f, spec.Qdiag, spec.Rdiag, dtype=dtype,
                  **spec.constraints)
+
+
+def digest(a):
+    """First 128 bits of the SHA-256 of an array's dtype, shape and bytes: comparing digests is a bit-for-bit comparison
+    (bits_equal) against an array that need not be stored."""
+    a = np.ascontiguousarray(a)
+    h = hashlib.sha256(f"{a.dtype.str}{a.shape}".encode())
+    h.update(a.tobytes())
+    return h.hexdigest()[:32]
+
+
+def stored_setup(store, prefix, index=None):
+    """A setup like oracle.ref_setup whose Q, R and cache are the ones the reference's tiny_setup computed, read from `store`
+    (a golden .npz) as <prefix>_<field>, or as row `index` of it."""
+    def setup(nx, nu, N, rho, A, B, f, Qdiag, Rdiag, dtype=np.float64, **constraints) -> MPCProblem:
+        dt = np.dtype(dtype).type
+        cache = {k: store[f"{prefix}_{k}"] if index is None else store[f"{prefix}_{k}"][index] for k in CACHE_FIELDS}
+        return MPCProblem(nx=nx, nu=nu, N=N, dtype=dt, rho=float(dt(rho)), A=np.asfortranarray(A, dtype=dt),
+                          B=np.asfortranarray(np.asarray(B, dtype=dt).reshape(nx, nu)), f=np.ascontiguousarray(f, dtype=dt),
+                          **cache, **constraints)
+    return setup
+
+
+def load_reference(name):
+    return np.load(os.path.join(REF_DIR, name + ".npz"))
+
+
+def lti_sweep(dt):
+    """Randomised sweep over the compiled (nx, nu) pairs and short horizons (BASELINE config 5's generator) ->
+    [(key, spec, inst)]: warm-started three-step loops whose first x0 pushes the rollout into the box bounds."""
+    dims = [(4, 1), (4, 2), (4, 8), (6, 3), (8, 4), (12, 2), (12, 8), (16, 4), (16, 8)]
+    out = []
+    for n, (nx, nu) in enumerate(dims):
+        N = (3, 7, 12)[n % 3]
+        sp = wl.random_lti(nx, nu, N, seed=40 + n)
+        sp.settings.max_iter = 25
+        sp.settings.check_termination = 1 + n % 3
+        inst = wl.random_instances(5, nx, N, seed=70 + n, dtype=dt)
+        inst["x0"] = (3.0 * inst["x0"]).astype(dt)
+        out.append((f"{nx}_{nu}_{N}", sp, inst))
+    return out
+
+
+def precompute_models():
+    """[(nx, nu, [spec])]: the models whose tiny_setup cache the device precompute is checked against."""
+    return [(12, 4, [wl.quadrotor(N=10), wl.quadrotor(N=10, hz=50)] + [wl.random_lti(12, 4, 10, seed=i) for i in range(6)]),
+            (6, 3, [wl.rocket(N=10)] + [wl.random_lti(6, 3, 10, seed=i) for i in range(5)]),
+            (16, 8, [wl.random_lti(16, 8, 10, seed=i) for i in range(6)])]
+
+
+EXAMPLES = ["cartpole_example", "quadrotor_hovering", "quadrotor_tracking", "rocket_landing_mpc", "quadrotor_linear_constraints",
+            "quadrotor_tv_linear_constraints"]
 
 
 def quad_linear_spec(tv=False, N=10):

@@ -1,9 +1,11 @@
-"""bench.py contract pieces that do not need a GPU: the algorithmic byte / flop counts of SURVEY §8(d), the host-core probe,
-and the reference arm's JSON line (run on a tiny sample)."""
+"""bench.py contract pieces: without a GPU, the algorithmic byte / flop counts of SURVEY §8(d), the host-core probe and the
+reference arm's JSON line (run on a tiny sample); on the GPU, the arrays --dump-outputs writes."""
 import json
 import os
 import subprocess
 import sys
+
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -39,3 +41,26 @@ def test_reference_arm_line():
     cb = d["cpu_baseline"]
     assert cb["kind"] in ("reference", "port") and cb["cores"] >= 1 and cb["one_thread"] > 0 and cb["value"] == d["value"]
     assert d["e2e"]["h2d_bytes_per_step"] == 0 and d["e2e"]["d2h_bytes_per_step"] == 0
+
+
+@pytest.mark.gpu
+def test_dump_outputs_writes_the_timed_solution(tmp_path):
+    """--dump-outputs writes, after the timed steps, the headline solve's arrays (a fixed sample of its instances) as
+    float32/float64 .npy files; they equal the oracle's solve of the same instances bit for bit."""
+    import numpy as np
+
+    from oracle import oracle
+    from tinympc_b200.solver import setup_problem
+
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "1", "--no-extras", "--no-cpu-baseline",
+                        "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=900)
+    assert r.returncode == 0, r.stderr[-2000:]
+    assert json.loads(r.stdout.strip().splitlines()[-1])["steps"] == 2
+    got = {k: np.load(tmp_path / f"C2_{k}.npy") for k in bench.DUMP_KEYS}
+    assert sorted(os.listdir(tmp_path)) == sorted(f"C2_{k}.npy" for k in bench.DUMP_KEYS)
+    assert all(a.dtype in (np.float32, np.float64) and a.shape[0] == bench.DUMP_INSTANCES for a in got.values())
+    case = bench.make_case("C2", B=bench.DUMP_INSTANCES)  # identical instances: any sample of the batch is this batch
+    prob = setup_problem(case["spec"], case["dtype"])
+    ref = oracle.solve_batch(prob, case["spec"].settings, case["inst"]["x0"], case["inst"]["Xref"], None, cold_start=True, nthreads=4)
+    for k in bench.DUMP_KEYS:
+        assert np.array_equal(got[k], ref[k].astype(got[k].dtype)), k

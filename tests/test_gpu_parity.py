@@ -558,19 +558,16 @@ def test_full_size_rocket_sample_vs_oracle():
 
 @pytest.mark.parametrize("dt", [np.float32, np.float64])
 def test_device_precompute_vs_reference_tiny_setup(dt):
-    """SURVEY §8f-2 against the REFERENCE: the device precompute's blobs vs tiny_setup of the compiled reference
-    (oracle.ref_setup -> tiny_api.cpp:21-147,307-381), per model.  fp64: <= 1e-9 of the matrix's largest entry (measured
+    """SURVEY §8f-2 against the REFERENCE: the device precompute's blobs vs the cache the compiled reference's tiny_setup
+    computed (tiny_api.cpp:21-147,307-381; stored in tests/golden/ by tests/golden/make_golden.py), per model.  fp64: <= 1e-9 of the matrix's largest entry (measured
     5e-14); fp32: <= 2e-5 where the Riccati fixed point converges in float (measured worst 1.1e-5: ~150 sweeps of fp32
     rounding under a 1e-5 stopping rule), <= 1e-4 where it never does (quadrotor 20 Hz: 1000 sweeps of a rounding-level limit
     cycle, measured 4.6e-5 — Eigen's inverse and the product's Gauss-Jordan differ in the last bits of every sweep)."""
     import torch
     from tinympc_b200.solver import unpack_model
 
-    if not oracle.ref_available(dt):
-        pytest.skip("compiled reference not present")
-    for nx, nu, specs in ((12, 4, [wl.quadrotor(N=10), wl.quadrotor(N=10, hz=50)] + [wl.random_lti(12, 4, 10, seed=i) for i in range(6)]),
-                          (6, 3, [wl.rocket(N=10)] + [wl.random_lti(6, 3, 10, seed=i) for i in range(5)]),
-                          (16, 8, [wl.random_lti(16, 8, 10, seed=i) for i in range(6)])):
+    gold = H.load_reference(f"tiny_setup_{np.dtype(dt).name}")
+    for nx, nu, specs in H.precompute_models():
         prob = setup_problem(specs[0], dt)
         solver = _mk_solver(prob, specs[0].settings, "auto")
         args = (np.stack([s.A for s in specs]), np.stack([np.asarray(s.B).reshape(nx, nu) for s in specs]), np.stack([s.f for s in specs]),
@@ -579,7 +576,7 @@ def test_device_precompute_vs_reference_tiny_setup(dt):
         torch.cuda.synchronize()
         dev, sweeps = dev.cpu().numpy(), sweeps.cpu().numpy()
         for i, sp in enumerate(specs):
-            ref = H.problem_from_spec(sp, dt, oracle.ref_setup)
+            ref = H.problem_from_spec(sp, dt, H.stored_setup(gold, f"{nx}_{nu}", i))
             m = unpack_model(dev[i], nx, nu)
             tol = 1e-9 if dt == np.float64 else (2e-5 if sweeps[i] < 1000 else 1e-4)
             for f in ("Q", "R", "Kinf", "Pinf", "Quu_inv", "AmBKt", "APf", "BPf"):

@@ -1,20 +1,21 @@
 """Drop-in check of the reference-compatible C++ front end (tinympc_b200/shim): the reference's OWN example
-programs (examples/*.cpp, compiled unmodified by tinympc_b200/shim/Makefile) are run twice — linked against the
-unmodified reference (CPU, pinned flags) and linked against the shim (B200) — and must print the same
-closed-loop results: every "tracking error" value, every iteration count, every "Solver converged" line.
-(The setup banner prints cache matrices with 4 significant digits and is compared too.)"""
+programs (examples/*.cpp, compiled unmodified by oracle/Makefile) linked against the shim (B200) must print the same
+closed-loop results as the same programs linked against the unmodified reference (CPU, pinned flags), whose output is
+stored in tests/golden/reference/examples/: every "tracking error" value, every iteration count, every "Solver converged"
+line.  (The setup banner prints cache matrices with 4 significant digits and is compared too.)"""
+import gzip
 import os
 import subprocess
 
 import pytest
 
+import helpers as H
+
 pytestmark = pytest.mark.gpu
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.path.join(ROOT, "oracle", "_ref", "examples_ref")
-SHIM = os.path.join(ROOT, "oracle", "_ref", "examples_shim")
-EXAMPLES = ["cartpole_example", "quadrotor_hovering", "quadrotor_tracking", "rocket_landing_mpc",
-            "quadrotor_linear_constraints", "quadrotor_tv_linear_constraints"]
+SHIM = os.path.join(ROOT, "oracle", "_ref", "shim_examples")
+KEYS = ("tracking error", "terations", "converged", "Tracking", "Average")
 
 
 def _run(path):
@@ -23,13 +24,15 @@ def _run(path):
     return r.stdout.splitlines()
 
 
-@pytest.mark.parametrize("name", EXAMPLES)
+@pytest.mark.parametrize("name", H.EXAMPLES)
 def test_reference_example_prints_identical_results_through_the_shim(name):
-    if not (os.path.exists(os.path.join(REF, name)) and os.path.exists(os.path.join(SHIM, name))):
-        pytest.skip("example binaries not prebuilt (tinympc_b200/shim/Makefile needs /root/reference)")
-    ref, shim = _run(os.path.join(REF, name)), _run(os.path.join(SHIM, name))
-    key = [ln for ln in ref if any(t in ln for t in ("tracking error", "terations", "converged", "Tracking", "Average"))]
-    key_s = [ln for ln in shim if any(t in ln for t in ("tracking error", "terations", "converged", "Tracking", "Average"))]
+    if not os.path.exists(os.path.join(SHIM, name)):
+        pytest.skip("example binaries not built (oracle/Makefile compiles them from the reference's sources)")
+    with gzip.open(os.path.join(H.REF_DIR, "examples", name + ".txt.gz"), "rt") as fh:
+        ref = fh.read().splitlines()
+    shim = _run(os.path.join(SHIM, name))
+    key = [ln for ln in ref if any(t in ln for t in KEYS)]
+    key_s = [ln for ln in shim if any(t in ln for t in KEYS)]
     assert len(key) > 10
     assert key == key_s, next((a, b) for a, b in zip(key, key_s) if a != b)
     assert ref == shim or len(ref) == len(shim)

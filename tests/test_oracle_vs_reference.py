@@ -1,7 +1,9 @@
 """The C restatement (oracle/tinympc_oracle.c) must be BIT-IDENTICAL to the unmodified reference compiled
-with the pinned flags (oracle/_ref/libtinympc_ref_{f64,f32}.so) on every parity case, through warm-started
-closed loops.  Runs only where the reference library exists (the build container; it is prebuilt and travels
-to the GPU box too)."""
+with the pinned flags on every parity case, through warm-started closed loops.  The reference's outputs (and the cache
+its tiny_setup computed) are stored in tests/golden/ by tests/golden/make_golden.py; here the port runs the cases
+from their definitions (tests/helpers.py), simulating the plant itself, and must reproduce them."""
+import os
+
 import numpy as np
 import pytest
 
@@ -20,29 +22,26 @@ def _solve(impl):
 @pytest.mark.parametrize("name", sorted(CASES))
 def test_port_bit_identical_to_reference(name):
     c = CASES[name]
-    if not oracle.ref_available(c["dtype"]):
-        pytest.skip("oracle/_ref not built (no /root/reference here)")
-    prob = H.problem_from_spec(c["spec"], c["dtype"], oracle.ref_setup)
+    gold = np.load(os.path.join(H.GOLDEN_DIR, name + ".npz"))
+    prob = H.problem_from_spec(c["spec"], c["dtype"], H.stored_setup(gold, "prob"))
     st = c["spec"].settings
-    ref, x0s = H.closed_loop(prob, st, c["inst"], c["steps"], c["reset_duals"], c["state"], _solve("reference"))
-    port, _ = H.closed_loop(prob, st, c["inst"], c["steps"], c["reset_duals"], c["state"], _solve("port"), x0_seq=x0s)
+    port, x0s = H.closed_loop(prob, st, c["inst"], c["steps"], c["reset_duals"], c["state"], _solve("port"))
+    assert H.bits_equal(np.stack(x0s), gold["x0_seq"])
     moved = 0
-    for k, (r, p) in enumerate(zip(ref, port)):
+    for k, p in enumerate(port):
         for key in H.OUT_KEYS + c["state"]:
-            assert H.bits_equal(r[key], p[key]), f"{name} step {k}: {key} differs"
-        moved += int(r["iter"].sum())
+            assert H.bits_equal(gold[f"step{k}_{key}"], p[key]), f"{name} step {k}: {key} differs"
+        moved += int(p["iter"].sum())
     assert moved > 0
 
 
 def test_precompute_port_close_to_reference():
     for name in ("cartpole_f64", "quad_hover_N10_f64", "rocket_soc_N10_f64", "lti_8_2_f64"):
         c = CASES[name]
-        if not oracle.ref_available(np.float64):
-            pytest.skip("oracle/_ref not built")
-        pr = H.problem_from_spec(c["spec"], np.float64, oracle.ref_setup)
+        gold = np.load(os.path.join(H.GOLDEN_DIR, name + ".npz"))
         pp = H.problem_from_spec(c["spec"], np.float64, oracle.port_setup)
-        for f in ("Kinf", "Pinf", "Quu_inv", "AmBKt", "APf", "BPf", "Q", "R"):
-            a, b = getattr(pr, f), getattr(pp, f)
+        for f in H.CACHE_FIELDS:
+            a, b = gold["prob_" + f], getattr(pp, f)
             assert np.allclose(a, b, rtol=1e-9, atol=1e-9 * max(1.0, np.abs(a).max())), (name, f)
 
 
@@ -50,21 +49,12 @@ def test_precompute_port_close_to_reference():
 def test_port_bit_identical_to_reference_random_lti_sweep(dt):
     """Randomised sweep over the compiled (nx, nu) pairs and short horizons (BASELINE config 5's generator): warm-started
     three-step loops with active box bounds, restatement vs the unmodified reference, bit for bit."""
-    from tinympc_b200 import workloads as wl
-
-    if not oracle.ref_available(dt):
-        pytest.skip("oracle/_ref not built (no /root/reference here)")
-    dims = [(4, 1), (4, 2), (4, 8), (6, 3), (8, 4), (12, 2), (12, 8), (16, 4), (16, 8)]
-    for n, (nx, nu) in enumerate(dims):
-        N = (3, 7, 12)[n % 3]
-        sp = wl.random_lti(nx, nu, N, seed=40 + n)
-        sp.settings.max_iter = 25
-        sp.settings.check_termination = 1 + n % 3
-        inst = wl.random_instances(5, nx, N, seed=70 + n, dtype=dt)
-        inst["x0"] = (3.0 * inst["x0"]).astype(dt)  # push the rollout into the bounds
-        prob = H.problem_from_spec(sp, dt, oracle.ref_setup)
-        ref, x0s = H.closed_loop(prob, sp.settings, inst, 3, False, H.BOX_STATE, _solve("reference"))
-        port, _ = H.closed_loop(prob, sp.settings, inst, 3, False, H.BOX_STATE, _solve("port"), x0_seq=x0s)
-        for k, (r, p) in enumerate(zip(ref, port)):
-            for key in H.OUT_KEYS + H.BOX_STATE:
-                assert H.bits_equal(r[key], p[key]), f"({nx},{nu},{N}) step {k}: {key} differs"
+    gold = H.load_reference(f"lti_sweep_{np.dtype(dt).name}")
+    want = dict(zip(gold["names"], gold["digests"]))
+    for key, sp, inst in H.lti_sweep(dt):
+        prob = H.problem_from_spec(sp, dt, H.stored_setup(gold, key))
+        port, x0s = H.closed_loop(prob, sp.settings, inst, 3, False, H.BOX_STATE, _solve("port"))
+        assert H.digest(np.stack(x0s)) == want[f"{key}_x0_seq"], key
+        for k, p in enumerate(port):
+            for name in H.OUT_KEYS + H.BOX_STATE:
+                assert H.digest(p[name]) == want[f"{key}_step{k}_{name}"], f"{key} step {k}: {name} differs"

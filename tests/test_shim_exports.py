@@ -1,6 +1,6 @@
 """The reference-compatible C++ front end (tinympc_b200/shim): every function the reference's headers define for the solve
 path is exported with C linkage (tiny_api.hpp:10-62, admm.hpp:9-34), and tiny_initialize_sensitivity_matrices leaves in the
-cache exactly what the reference's does (tiny_api.cpp:479-540).  No GPU needed (nothing is solved)."""
+cache exactly what the reference's does (tiny_api.cpp:479-540, stored in tests/golden/).  No GPU needed (nothing is solved)."""
 import ctypes as C
 import os
 import subprocess
@@ -8,7 +8,7 @@ import subprocess
 import numpy as np
 import pytest
 
-from oracle import oracle
+import helpers as H
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 SHIM = os.path.join(ROOT, "tinympc_b200", "lib", "libtinympc_shim.so")
@@ -30,12 +30,11 @@ def test_shim_exports_the_reference_interface():
 
 
 def test_sensitivity_tables_equal_the_reference():
-    if not oracle.ref_available(np.float64):
-        pytest.skip("compiled reference not present")
+    """Against the tables the reference's tiny_initialize_sensitivity_matrices leaves (tests/golden/make_golden.py)."""
+    gold = H.load_reference("sensitivity_tables")
     shapes = [(4, 12), (12, 12), (4, 4), (12, 12)]
-    ref = [np.zeros(s, np.float64, order="F") for s in shapes]
-    rc = oracle.ref_lib(np.float64).tinympc_ref_sensitivity_tables(*[C.c_void_p(a.ctypes.data) for a in ref])
-    assert rc == 0
+    ref = [np.asfortranarray(gold[n]) for n in ("dKinf_drho", "dPinf_drho", "dC1_drho", "dC2_drho")]
+    assert [a.shape for a in ref] == shapes
     lib = C.CDLL(SHIM)
     mine = [np.zeros(s, np.float64, order="F") for s in shapes]
     assert lib.tinympc_shim_sensitivity_tables(*[C.c_void_p(a.ctypes.data) for a in mine]) == 0
