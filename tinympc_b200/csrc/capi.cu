@@ -133,11 +133,10 @@ struct tinympc_b200_solver {
     tinympc_settings_t settings;
     int mode = TINYMPC_MODE_STRICT;
     int family = TINYMPC_KERNEL_AUTO;
-    // workspace (one solve at a time per handle: enqueue() serialises launches issued on different streams)
-    DevBuf ws;
+    // launch scratch (one solve at a time per handle: enqueue() serialises launches issued on different streams)
+    DevBuf ws;          // TPI / GPS workspace
     DevBuf queue;
-    DevBuf vscratch;
-    DevBuf gps_ws;
+    DevBuf vscratch;    // GPI: work->v / work->z staging
     DevBuf shared_ref;  // host path: references shared by the whole batch
     cudaEvent_t ev_last = nullptr;  // recorded after the last enqueue
     cudaStream_t last_stream = nullptr;
@@ -159,6 +158,14 @@ int upload(DevBuf &b, const void *src, size_t n) {
     if (!src || n == 0) return 0;
     if (b.ensure(n)) return -1;
     return cudaMemcpy(b.p, src, n, cudaMemcpyHostToDevice) == cudaSuccess ? 0 : -1;
+}
+
+// grow a launch buffer of the handle to n bytes; the previous solve may still be using it, so wait for that one first
+int grow(tinympc_b200_solver *s, DevBuf &b, size_t n, const char *what) {
+    if (n <= b.bytes) return 0;
+    if (s->have_last) CUDA_TRY(cudaEventSynchronize(s->ev_last));
+    if (b.ensure(n)) return fail(TINYMPC_ERR_CUDA, std::string(what) + " allocation failed");
+    return 0;
 }
 
 struct Features {
@@ -190,23 +197,15 @@ int check_ready(const tinympc_b200_solver *s) {
 
 // Which kernel family serves a solve.  GPI = lane groups, state on chip (box constraints, horizon fits in shared + tensor
 // memory); GPS = lane groups, state streamed (everything else the lane mapping covers); TPI = one thread per instance.
-// `smem_out`: shared-memory bytes of the on-chip plan (0 = not available).  Returns -1 when an explicit request cannot
-// be honoured.
-int resolve_family(const tinympc_b200_solver *s, const Features &ft, int *smem_out, int64_t B = 0) {
-    int smem = 0;
-    bool gpi_ok = false;
-    if (!ft.ext && s->dim->gpi_fit) {
-        smem = s->dim->gpi_fit(s->dtype, s->N, s->max_smem_optin);
-        gpi_ok = smem > 0;
-    }
-    if (smem_out) *smem_out = smem;
-    const bool gps_ok = s->dim->gps_lanes && s->dim->gps_lanes(s->dtype) > 0;
+// `gpi` / `gps`: the plans of the two lane-group families for this solve (family 0 = not available).  Returns -1 when an
+// explicit request cannot be honoured.
+int resolve_family(const tinympc_b200_solver *s, const Features &ft, const tmpc::LaunchPlan &gpi, const tmpc::LaunchPlan &gps, int64_t B) {
+    const bool gpi_ok = gpi.family != 0, gps_ok = gps.family != 0;
     if (s->family == TINYMPC_KERNEL_GPI) return gpi_ok ? TINYMPC_KERNEL_GPI : (gps_ok ? TINYMPC_KERNEL_GPS : -1);
     if (s->family == TINYMPC_KERNEL_GPS) return gps_ok ? TINYMPC_KERNEL_GPS : -1;
     if (s->family == TINYMPC_KERNEL_TPI) return TINYMPC_KERNEL_TPI;
     // AUTO (measured rules; evidence: profiles/r02_auto_rule_sweep.md, profiles/r01_sweep_1gpu.md)
-    const int gps_plan = gps_ok ? s->dim->gps_lanes(s->dtype) : 0;
-    const bool gps_two = ((gps_plan >> 8) & 0xff) == 2;  // two instances per lane group: the small shapes
+    const bool gps_two = gps.group_instances == 2;  // two instances per lane group: the small shapes
     const bool big_batch = B >= (int64_t)s->sm_count * 384;  // one thread per instance fills the GPU
     // cones / hyperplanes: streamed lane groups (rocket landing, fp64: 3.3x the thread-per-instance kernel)
     if (ft.ext) return gps_ok ? TINYMPC_KERNEL_GPS : TINYMPC_KERNEL_TPI;
@@ -221,8 +220,7 @@ int resolve_family(const tinympc_b200_solver *s, const Features &ft, int *smem_o
     // AND the batch is large.  Measured on B200 (B = 131 072, N = 100): at 16 instances/SM the streamed kernels win by 10-35 %
     // for every shape except (16,8), where the thread-per-instance register footprint costs more than the low on-chip
     // occupancy; at >= 32 instances/SM GPI always wins.
-    const int plan = s->dim->gpi_instances_per_cta ? s->dim->gpi_instances_per_cta(s->dtype, s->N, s->max_smem_optin) : 0;
-    const int ipc = plan & 0xffff, gpi_warps = plan >> 16;
+    const int ipc = gpi.instances_per_cta, gpi_warps = gpi.warps_resident;
     if (s->dtype == TINYMPC_F64) {
         // fp64 (rows re-read per sweep, duals in tensor memory): on chip wins as soon as four warps per SM are resident
         // ((12,4,50): 29.6 vs 35.9 ms TPI at 16 instances/SM; (16,8,50): 57.3 vs 88.4 ms at 8/SM), and loses badly with one
@@ -235,42 +233,11 @@ int resolve_family(const tinympc_b200_solver *s, const Features &ft, int *smem_o
     return TINYMPC_KERNEL_GPI;
 }
 
-// carve the TPI structure-of-arrays workspace
-int setup_workspace(tinympc_b200_solver *s, tmpc::LaunchDesc &d, const Features &ft, int64_t B, int family) {
-    const int64_t Bpad = (B + 31) / 32 * 32;
-    d.Bpad = Bpad;
-    if (family != TINYMPC_KERNEL_TPI) return 0;
-    const int E = s->dtype == TINYMPC_F64 ? 2 : 4;
-    const size_t nxv = (s->nx + E - 1) / E, nuv = (s->nu + E - 1) / E;
-    const size_t szx = (size_t)s->N * nxv * 16 * Bpad, szu = (size_t)(s->N - 1) * nuv * 16 * Bpad;
-    size_t total = 3 * szx + 4 * szu;
-    if (ft.soc_x) total += 2 * szx;
-    if (ft.soc_u) total += 2 * szu;
-    if (ft.lin_x) total += 2 * szx;
-    if (ft.lin_u) total += 2 * szu;
-    if (ft.tvl_x) total += 2 * szx;
-    if (ft.tvl_u) total += 2 * szu;
-    if (s->ws.ensure(total + 256)) return fail(TINYMPC_ERR_CUDA, "workspace allocation failed");
-    char *c = (char *)s->ws.p;
-    auto take = [&](size_t n) {
-        void *r = c;
-        c += n;
-        return r;
-    };
-    d.w_v[0] = take(szx); d.w_v[1] = take(szx); d.w_g = take(szx);
-    d.w_z[0] = take(szu); d.w_z[1] = take(szu); d.w_y = take(szu); d.w_d = take(szu);
-    d.w_vc = d.w_gc = d.w_zc = d.w_yc = d.w_vl = d.w_gl = d.w_zl = d.w_yl = d.w_vlt = d.w_glt = d.w_zlt = d.w_ylt = nullptr;
-    if (ft.soc_x) { d.w_vc = take(szx); d.w_gc = take(szx); }
-    if (ft.soc_u) { d.w_zc = take(szu); d.w_yc = take(szu); }
-    if (ft.lin_x) { d.w_vl = take(szx); d.w_gl = take(szx); }
-    if (ft.lin_u) { d.w_zl = take(szu); d.w_yl = take(szu); }
-    if (ft.tvl_x) { d.w_vlt = take(szx); d.w_glt = take(szx); }
-    if (ft.tvl_u) { d.w_zlt = take(szu); d.w_ylt = take(szu); }
-    return 0;
-}
-
-void base_desc(const tinympc_b200_solver *s, tmpc::LaunchDesc &d, const Features &ft) {
+// the launch descriptor of a solve of `io` on the handle's problem
+void base_desc(const tinympc_b200_solver *s, tmpc::LaunchDesc &d, const Features &ft, const tinympc_batch_t &io) {
     std::memset(&d, 0, sizeof(d));
+    d.io = io;
+    d.Bpad = (io.B + 31) / 32 * 32;
     d.dtype = s->dtype;
     d.fast = s->mode == TINYMPC_MODE_FAST;
     d.ext = ft.ext;
@@ -299,43 +266,7 @@ void base_desc(const tinympc_b200_solver *s, tmpc::LaunchDesc &d, const Features
     d.h_xlo = s->h_xlo.empty() ? nullptr : s->h_xlo.data(); d.h_xhi = s->h_xhi.empty() ? nullptr : s->h_xhi.data();
     d.h_ulo = s->h_ulo.empty() ? nullptr : s->h_ulo.data(); d.h_uhi = s->h_uhi.empty() ? nullptr : s->h_uhi.data();
     d.sm_count = s->sm_count;
-    d.max_smem_optin = s->max_smem_optin;
-}
-
-// view of a (device) batch restricted to instances [b0, b0+nb)
-tinympc_batch_t slice_batch(const tinympc_b200_solver *s, const tinympc_batch_t &io, int64_t b0, int64_t nb) {
-    const size_t es = esize(s->dtype);
-    const size_t bx = es * s->nx * s->N, bu = es * s->nu * (s->N - 1);
-    tinympc_batch_t o = io;
-    o.B = nb;
-    auto adv = [&](const void *p, size_t per) -> void * { return p ? (void *)((const char *)p + per * (size_t)b0) : nullptr; };
-    o.x0 = adv(io.x0, es * s->nx);
-    if (io.xref_per_instance) o.Xref = adv(io.Xref, bx);
-    if (io.uref_per_instance) o.Uref = adv(io.Uref, bu);
-    void *const *sp = (void *const *)&io.state;
-    void **dp = (void **)&o.state;
-    const int nfields = sizeof(tinympc_state_t) / sizeof(void *);
-    for (int i = 0; i < nfields; ++i) dp[i] = adv(sp[i], (i % 2) == 0 ? bx : bu);
-    o.sol_x = adv(io.sol_x, bx);
-    o.sol_u = adv(io.sol_u, bu);
-    o.iter = (int32_t *)adv(io.iter, sizeof(int32_t));
-    o.solved = (int32_t *)adv(io.solved, sizeof(int32_t));
-    o.residuals = adv(io.residuals, 4 * es);
-    o.u0 = adv(io.u0, es * s->nu);
-    o.models = adv(io.models, es * (size_t)tinympc_b200_model_blob_elems(s->nx, s->nu));
-    return o;
-}
-
-// TPI streams its per-instance state through global memory every iteration.  TINYMPC_TPI_CHUNK=<n> solves
-// the batch in sub-batches of n instances (an experiment knob: an L2-sized working set did NOT pay off).
-int64_t tpi_chunk_instances(const tinympc_b200_solver *s, const Features &ft, int64_t B) {
-    if (const char *e = std::getenv("TINYMPC_TPI_CHUNK")) {
-        long long v = std::atoll(e);
-        if (v > 0) return std::min<int64_t>(B, (v + 127) / 128 * 128);
-        if (v < 0) return B;  // chunking off
-    }
-    (void)ft;
-    return B;  // measured on B200 (profiles/r01_tpi_chunk_sweep.txt): sub-batching only lowers occupancy; TPI is latency-, not L2-, limited
+    d.smem_budget = s->max_smem_optin - 64;
 }
 
 // enqueue one batched solve on `stream` (device pointers); fills stats
@@ -344,85 +275,51 @@ int enqueue(tinympc_b200_solver *s, const tinympc_batch_t *io, cudaStream_t stre
     if (!io->x0 || !io->Xref) return fail(TINYMPC_ERR_ARG, "x0 and Xref are required");
     if (io->B <= 0) return TINYMPC_OK;
     const Features ft = features(s);
-    int smem = 0;
-    int family = resolve_family(s, ft, &smem, io->B);
+    tmpc::LaunchDesc d;
+    base_desc(s, d, ft, *io);
+    d.stream = stream;
+    const tmpc::LaunchPlan gpi = s->dim->plan(d, TINYMPC_KERNEL_GPI), gps = s->dim->plan(d, TINYMPC_KERNEL_GPS);
+    int family = resolve_family(s, ft, gpi, gps, io->B);
     if (io->models) {  // per-instance models: on-chip kernel only
-        if (ft.ext || smem <= 0 || s->family == TINYMPC_KERNEL_TPI || s->family == TINYMPC_KERNEL_GPS)
+        if (!gpi.family || s->family == TINYMPC_KERNEL_TPI || s->family == TINYMPC_KERNEL_GPS)
             return fail(TINYMPC_ERR_UNSUPPORTED, "per-instance models need the on-chip GPI kernel (box constraints, horizon fitting in shared memory)");
         family = TINYMPC_KERNEL_GPI;
     }
     if (family < 0) return fail(TINYMPC_ERR_UNSUPPORTED, "the requested lane-group kernel does not cover this problem shape");
+    const tmpc::LaunchPlan plan = family == TINYMPC_KERNEL_GPI ? gpi : family == TINYMPC_KERNEL_GPS ? gps : s->dim->plan(d, family);
+    if (!plan.family) return fail(TINYMPC_ERR_UNSUPPORTED, "no compiled kernel for this (dtype, mode, family) combination");
     // The launch scratch of a handle (work queue, workspaces, timing events) is single-buffered: a solve enqueued on a
     // different stream than the previous one first waits for it.
     if (s->have_last && s->last_stream != stream) CUDA_TRY(cudaStreamWaitEvent(stream, s->ev_last, 0));
-    int64_t launches = 0, ctas = 0;
-    size_t ws_bytes = 0;
-    tmpc::LaunchDesc d;
-    base_desc(s, d, ft);
+    if (int rc = grow(s, s->ws, plan.workspace_bytes, "workspace")) return rc;
+    if (int rc = grow(s, s->vscratch, plan.scratch_bytes, "GPI v-scratch")) return rc;
+    d.workspace = s->ws.p;
+    d.scratch = plan.scratch_bytes ? s->vscratch.p : nullptr;
     if (timed) CUDA_TRY(cudaEventRecord(s->ev0, stream));
-    d.family = family;
-    d.stream = stream;
-    if (family == TINYMPC_KERNEL_GPI || family == TINYMPC_KERNEL_GPS) {
+    if (family != TINYMPC_KERNEL_TPI) {
         if (s->queue.ensure(256)) return fail(TINYMPC_ERR_CUDA, "queue allocation failed");
         CUDA_TRY(cudaMemsetAsync(s->queue.p, 0, 256, stream));
         d.work_queue = s->queue.p;
-        d.gpi_vscratch = nullptr;
-        if (family == TINYMPC_KERNEL_GPI && (io->state.v || io->state.z)) {  // previous-iteration slacks are staged in pack layout, one 16-byte store per knot point
-            const int plan = s->dim->gpi_instances_per_cta(s->dtype, s->N, s->max_smem_optin);
-            const int warps = plan >> 16, ipc = plan & 0xffff;
-            const int L = (warps > 0 && ipc > 0) ? 32 * warps / ipc : 4;
-            const int W = s->dtype == TINYMPC_F64 ? 2 : 4;
-            const int pv = (s->nx + L - 1) / L + (s->nu + L - 1) / L;
-            const size_t pvp = (size_t)(pv + W - 1) / W * W;
-            if (s->vscratch.ensure((size_t)io->B * s->N * L * pvp * esize(s->dtype) + 256)) return fail(TINYMPC_ERR_CUDA, "GPI v-scratch allocation failed");
-            d.gpi_vscratch = s->vscratch.p;
-        }
-        d.Bpad = (io->B + 31) / 32 * 32;
-        d.io = *io;
-        d.gps_ws = s->gps_ws.p;
-        d.gps_ws_bytes = s->gps_ws.bytes;
-        int rc = s->dim->launch(&d);
-        if (rc == tmpc::TM_ERR_WORKSPACE) {  // the streamed kernel sizes its workspace by resident slots: grow and retry
-            if (s->have_last) CUDA_TRY(cudaEventSynchronize(s->ev_last));  // a previous solve may still use the old buffer
-            if (s->gps_ws.ensure(d.out_ws_need + 256)) return fail(TINYMPC_ERR_CUDA, "GPS workspace allocation failed");
-            d.gps_ws = s->gps_ws.p;
-            d.gps_ws_bytes = s->gps_ws.bytes;
-            rc = s->dim->launch(&d);
-        }
-        if (rc == TINYMPC_ERR_CUDA) return fail(rc, std::string("kernel launch failed: ") + cudaGetErrorString(cudaGetLastError()));
-        if (rc) return fail(TINYMPC_ERR_UNSUPPORTED, "no compiled kernel for this (dtype, mode, family) combination");
-        ++launches;
-        ctas += d.out_ctas;
-        if (family == TINYMPC_KERNEL_GPS) ws_bytes = d.out_ws_need;
-    } else {
-        const int64_t chunk = tpi_chunk_instances(s, ft, io->B);
-        if (int rc = setup_workspace(s, d, ft, chunk, TINYMPC_KERNEL_TPI)) return rc;
-        ws_bytes = s->ws.bytes;
-        for (int64_t b0 = 0; b0 < io->B; b0 += chunk) {
-            d.io = slice_batch(s, *io, b0, std::min<int64_t>(chunk, io->B - b0));
-            int rc = s->dim->launch(&d);
-            if (rc == TINYMPC_ERR_CUDA) return fail(rc, std::string("kernel launch failed: ") + cudaGetErrorString(cudaGetLastError()));
-            if (rc) return fail(rc, "no compiled kernel for this (dtype, mode, family) combination");
-            ++launches;
-            ctas += d.out_ctas;
-        }
     }
-    s->stats.lanes_per_instance = d.out_lanes_per_instance;
-    s->stats.instances_per_cta = d.out_instances_per_cta;
-    s->stats.smem_bytes_per_cta = d.out_smem;
-    s->stats.threads_per_cta = d.out_threads;
-    s->stats.tmem_cols_per_cta = d.out_tmem_cols;
+    const int rc = s->dim->launch(&d, plan);
+    if (rc == TINYMPC_ERR_CUDA) return fail(rc, std::string("kernel launch failed: ") + cudaGetErrorString(cudaGetLastError()));
+    if (rc) return fail(rc, "no compiled kernel for this (dtype, mode, family) combination");
     if (timed) CUDA_TRY(cudaEventRecord(s->ev1, stream));
     CUDA_TRY(cudaEventRecord(s->ev_last, stream));
     s->last_stream = stream;
     s->have_last = true;
     s->timed = timed;
     s->stats.instances = io->B;
-    s->stats.kernel_launches = launches;
+    s->stats.kernel_launches = 1;
     s->stats.kernel_family = family;
-    s->stats.ctas = (int)ctas;
+    s->stats.lanes_per_instance = plan.lanes;
+    s->stats.instances_per_cta = plan.instances_per_cta;
+    s->stats.smem_bytes_per_cta = (int)plan.smem;
+    s->stats.threads_per_cta = plan.threads;
+    s->stats.tmem_cols_per_cta = plan.tmem_cols;
+    s->stats.ctas = plan.ctas;
     s->stats.gpi_instances = family == TINYMPC_KERNEL_TPI ? 0 : io->B;
-    s->stats.workspace_bytes = (int64_t)ws_bytes;
+    s->stats.workspace_bytes = (int64_t)plan.workspace_bytes;
     return TINYMPC_OK;
 }
 
@@ -657,7 +554,7 @@ int tinympc_b200_destroy(tinympc_b200_solver_t *s) {
     cudaSetDevice(s->device);
     DevBuf *bufs[] = {&s->d_xmin, &s->d_xmax, &s->d_umin, &s->d_umax, &s->d_Alin_x, &s->d_blin_x, &s->d_Alin_u,
                       &s->d_blin_u, &s->d_tvA_x, &s->d_tvb_x, &s->d_tvA_u, &s->d_tvb_u, &s->ws, &s->queue, &s->d_blob, &s->vscratch,
-                      &s->gps_ws, &s->shared_ref};
+                      &s->shared_ref};
     for (DevBuf *b : bufs) b->release();
     for (int i = 0; i < tinympc_b200_solver::SLOTS; ++i) {
         s->dio[i].release();
@@ -799,8 +696,7 @@ int tinympc_b200_solve_host(tinympc_b200_solver_t *s, const tinympc_batch_t *io)
     {
         size_t need = (io->xref_per_instance ? 0 : bx) + ((io->Uref && !io->uref_per_instance) ? bu : 0);
         if (need) {
-            if (need + 256 > shared_ref.bytes && s->have_last) CUDA_TRY(cudaEventSynchronize(s->ev_last));  // about to reallocate
-            if (shared_ref.ensure(need + 256)) return fail(TINYMPC_ERR_CUDA, "shared reference allocation failed");
+            if (int rc = grow(s, shared_ref, need + 256, "shared reference")) return rc;
             char *c = (char *)shared_ref.p;
             if (!io->xref_per_instance) {
                 CUDA_TRY(cudaMemcpyAsync(c, io->Xref, bx, cudaMemcpyHostToDevice, s->st_h2d));
@@ -831,12 +727,6 @@ int tinympc_b200_solve_host(tinympc_b200_solver_t *s, const tinympc_batch_t *io)
     if (io->residuals) fields.push_back({nullptr, io->residuals, 4 * es, false, true, (void **)&dev.residuals});
 
     for (Field &f : fields) f.pinned = is_pinned(f.is_out ? f.dst : f.src) && (!f.is_in || !f.src || is_pinned(f.src));
-    size_t per_inst_dev = 0, per_inst_in = 0, per_inst_out = 0;
-    for (const Field &f : fields) {
-        per_inst_dev += f.per_inst;
-        if (f.is_in) per_inst_in += f.per_inst;
-        if (f.is_out) per_inst_out += f.per_inst;
-    }
     // chunking: big enough to fill the GPU several times over, small enough to pipeline
     int64_t chunk = B;
     if (B > 16384) chunk = std::max<int64_t>(8192, (B + 7) / 8);
@@ -844,10 +734,13 @@ int tinympc_b200_solve_host(tinympc_b200_solver_t *s, const tinympc_batch_t *io)
     {   // the persistent GPI kernel holds sm_count * instances_per_cta instances at a time: make a chunk a whole
         // number of such waves so that no chunk ends on a mostly empty wave
         const Features ft = features(s);
-        int smem = 0;
-        const int fam = resolve_family(s, ft, &smem, chunk);
-        if (fam == TINYMPC_KERNEL_GPI && s->dim->gpi_instances_per_cta && B > 16384) {
-            const int64_t wave = (int64_t)s->sm_count * (s->dim->gpi_instances_per_cta(s->dtype, s->N, s->max_smem_optin) & 0xffff);
+        tinympc_batch_t first = *io;
+        first.B = chunk;
+        tmpc::LaunchDesc d;
+        base_desc(s, d, ft, first);
+        const tmpc::LaunchPlan gpi = s->dim->plan(d, TINYMPC_KERNEL_GPI);
+        if (B > 16384 && resolve_family(s, ft, gpi, s->dim->plan(d, TINYMPC_KERNEL_GPS), chunk) == TINYMPC_KERNEL_GPI) {
+            const int64_t wave = (int64_t)s->sm_count * gpi.instances_per_cta;
             if (wave > 0 && wave < B) chunk = std::max<int64_t>(1, (chunk + wave / 2) / wave) * wave;
         }
     }
@@ -946,7 +839,6 @@ int tinympc_b200_solve_host(tinympc_b200_solver_t *s, const tinympc_batch_t *io)
     s->stats.kernel_launches = launches;
     s->timed = false;
     s->stats.kernel_ms = 0.f;
-    (void)per_inst_dev; (void)per_inst_in; (void)per_inst_out;
     return TINYMPC_OK;
 }
 

@@ -1208,22 +1208,17 @@ __global__ void __launch_bounds__(GPI_MAX_WARPS * 32, 1)
 }
 
 // ---------------------------------------------------------------------------------------------------------
-// host side: configuration choice + launch
+// host side: plan + launch
 // ---------------------------------------------------------------------------------------------------------
-struct GpiPlan {
-    int L = 0, warps = 0;
-    size_t smem = 0;
-    bool tm = false;  // dual packs + d in tensor memory
-};
-
 // TINYMPC_GPI_TMEM=0 keeps everything in shared memory (A/B switch for measurements)
 inline bool gpi_allow_tm() {
     const char *e = std::getenv("TINYMPC_GPI_TMEM");
     return !(e && e[0] == '0');
 }
 
+// candidate (L, TM): replaces `best` (lanes, warps_resident, smem, tmem_cols) when it holds more; pvp = its GpiCfg::PVP
 template <typename T, int NX, int NU, int L, bool TM>
-inline void gpi_consider(int N, int max_smem, GpiPlan &best) {
+inline void gpi_consider(int N, int max_smem, LaunchPlan &best, int &pvp) {
     if constexpr (gpi_feasible<T, NX, NU, L>()) {
         using Cfg = GpiCfg<NX, NU, L, (int)sizeof(T)>;
         const size_t per_warp = (TM ? Cfg::warp_elems_tm(N) : Cfg::warp_elems(N)) * sizeof(T);
@@ -1241,20 +1236,24 @@ inline void gpi_consider(int N, int max_smem, GpiPlan &best) {
         }
         if (w < 1 || blob > (size_t)max_smem) return;
         // score: instances resident per SM, then fewer lanes per instance (less shuffle traffic)
-        const int inst = w * Cfg::IPW, binst = best.warps * (best.L ? 32 / best.L : 0);
-        const bool better = best.L == 0 || (w >= 4 && best.warps < 4) || (((w >= 4) == (best.warps >= 4)) && inst > binst);
+        const int inst = w * Cfg::IPW, binst = best.warps_resident * (best.lanes ? 32 / best.lanes : 0);
+        const bool better = best.lanes == 0 || (w >= 4 && best.warps_resident < 4) ||
+                            (((w >= 4) == (best.warps_resident >= 4)) && inst > binst);
         if (better) {
-            best.L = L;
-            best.warps = w;
+            best.lanes = L;
+            best.warps_resident = w;
             best.smem = std::max(keep + per_warp * (size_t)w, blob);
-            best.tm = TM;
+            best.tmem_cols = TM ? 512 : 0;  // the kernel allocates all of them
+            pvp = Cfg::PVP;
         }
     }
 }
 
 template <typename T, int NX, int NU>
-inline GpiPlan gpi_plan(int N, int max_smem) {
-    GpiPlan p;
+inline LaunchPlan gpi_plan(const LaunchDesc &d) {
+    LaunchPlan p;
+    int pvp = 0;
+    const int N = d.N, max_smem = d.smem_budget;
     // L = 16 is only ever needed in fp64 (two registers per matrix entry: L = 4 / 8 exceed the register ceiling from
     // nx = 12 on); for fp32 L = 8 covers every (nx, nu) pair of TM_DIMS, so the fp32 L = 16 kernels are compiled only
     // with -DTM_GPI_L16 (wider states) to keep the build short
@@ -1266,45 +1265,40 @@ inline GpiPlan gpi_plan(int N, int max_smem) {
     // TINYMPC_GPI_LANES=4|8|16 restricts the choice to one group width (A/B switch for measurements)
     const char *e = std::getenv("TINYMPC_GPI_LANES");
     const int only = e ? std::atoi(e) : 0;
-    if (!only || only == 4) gpi_consider<T, NX, NU, 4, false>(N, max_smem, p);
-    if (!only || only == 8) gpi_consider<T, NX, NU, 8, false>(N, max_smem, p);
+    if (!only || only == 4) gpi_consider<T, NX, NU, 4, false>(N, max_smem, p, pvp);
+    if (!only || only == 8) gpi_consider<T, NX, NU, 8, false>(N, max_smem, p, pvp);
     if constexpr (L16)
-        if (!only || only == 16) gpi_consider<T, NX, NU, 16, false>(N, max_smem, p);
+        if (!only || only == 16) gpi_consider<T, NX, NU, 16, false>(N, max_smem, p, pvp);
     if (gpi_allow_tm()) {  // taken only when it holds more instances per SM
-        if (!only || only == 4) gpi_consider<T, NX, NU, 4, true>(N, max_smem, p);
-        if (!only || only == 8) gpi_consider<T, NX, NU, 8, true>(N, max_smem, p);
+        if (!only || only == 4) gpi_consider<T, NX, NU, 4, true>(N, max_smem, p, pvp);
+        if (!only || only == 8) gpi_consider<T, NX, NU, 8, true>(N, max_smem, p, pvp);
         if constexpr (L16)
-            if (!only || only == 16) gpi_consider<T, NX, NU, 16, true>(N, max_smem, p);
+            if (!only || only == 16) gpi_consider<T, NX, NU, 16, true>(N, max_smem, p, pvp);
     }
+    if (p.lanes == 0) return p;
+    p.family = TINYMPC_KERNEL_GPI;
+    p.instances_per_cta = p.warps_resident * (32 / p.lanes);
+    const int64_t ngroups = (d.io.B + (32 / p.lanes) - 1) / (32 / p.lanes);
+    // ngroups = warps the batch fills.  A batch smaller than one wave is spread over all SMs with fewer warps per CTA
+    // (the kernel's carve-up is per warp, any block size up to warps_resident works): the latency of a solve is set by how
+    // many warps share a scheduler (C2: 2.08 ms per 100 iterations with 8 warps per SM, 1.34 ms with one).
+    int warps = p.warps_resident;
+    if ((ngroups + warps - 1) / warps < d.sm_count) warps = (int)std::max<int64_t>(1, (ngroups + d.sm_count - 1) / d.sm_count);
+    const int64_t want = (ngroups + warps - 1) / warps;
+    p.ctas = (int)std::max<int64_t>(1, std::min<int64_t>(d.sm_count, want));
+    p.threads = warps * 32;
+    // work->v / work->z persistence: the previous-iteration slacks are staged in pack layout, one 16-byte store per knot point
+    if (d.io.state.v || d.io.state.z) p.scratch_bytes = (size_t)d.io.B * N * p.lanes * pvp * sizeof(T) + 256;
     return p;
 }
 
-template <typename T, int NX, int NU>
-inline int gpi_fit_T(int N, int max_smem) {
-    return (int)gpi_plan<T, NX, NU>(N, max_smem).smem;
-}
-
 template <typename T, int NX, int NU, int L, bool FAST, bool HET, bool TM, bool MM = false>
-int launch_gpi_L(LaunchDesc *d, const GpiPlan &plan, const KParams<T, NX, NU> &P, const T *gmat) {
+int launch_gpi_L(LaunchDesc *d, const LaunchPlan &plan, const KParams<T, NX, NU> &P, const T *gmat) {
     if constexpr (gpi_feasible<T, NX, NU, L>()) {
         auto kern = gpi_solve_kernel<T, NX, NU, L, FAST, HET, TM, MM>;
         if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)plan.smem) != cudaSuccess)
             return TINYMPC_ERR_CUDA;
-        const int64_t ngroups = (d->io.B + (32 / L) - 1) / (32 / L);
-        // ngroups = warps the batch fills.  A batch smaller than one wave is spread over all SMs with fewer warps per CTA
-        // (the kernel's carve-up is per warp, any block size up to plan.warps works): the latency of a solve is set by how
-        // many warps share a scheduler (C2: 2.08 ms per 100 iterations with 8 warps per SM, 1.34 ms with one).
-        int warps = plan.warps;
-        if ((ngroups + warps - 1) / warps < d->sm_count) warps = (int)std::max<int64_t>(1, (ngroups + d->sm_count - 1) / d->sm_count);
-        const int64_t want = (ngroups + warps - 1) / warps;
-        const int ctas = (int)std::max<int64_t>(1, std::min<int64_t>(d->sm_count, want));
-        kern<<<ctas, warps * 32, plan.smem, d->stream>>>(P, gmat, (unsigned long long *)d->work_queue);
-        d->out_threads = warps * 32;
-        d->out_ctas = ctas;
-        d->out_smem = (int)plan.smem;
-        d->out_lanes_per_instance = L;
-        d->out_instances_per_cta = plan.warps * (32 / L);
-        d->out_tmem_cols = TM ? 512 : 0;
+        kern<<<plan.ctas, plan.threads, plan.smem, d->stream>>>(P, gmat, (unsigned long long *)d->work_queue);
         return cudaGetLastError() == cudaSuccess ? TINYMPC_OK : TINYMPC_ERR_CUDA;
     } else {
         return TINYMPC_ERR_UNSUPPORTED;

@@ -1185,67 +1185,53 @@ __global__ void __launch_bounds__(gps_max_warps(NI) * 32, 1)
 }
 
 // ---------------------------------------------------------------------------------------------------------
-// host side: record layout, resident-slot plan, launch
+// host side: resident-slot plan, variant dispatch, launch
 // ---------------------------------------------------------------------------------------------------------
-struct GpsPlan {
-    int L = 0, NI = 0, warps = 0, ctas = 0;
-    size_t smem = 0, ws_bytes = 0;
-    GpsLayout ly;
-};
-
 inline int gps_env_int(const char *name, int dflt) {
     const char *e = std::getenv(name);
     return e ? std::atoi(e) : dflt;
 }
 
 template <typename T, int NX, int NU, int L, int NI, int FAM>
-inline GpsPlan gps_plan_L(const LaunchDesc &d) {
+inline LaunchPlan gps_plan_L(const LaunchDesc &d) {
     using Cfg = GpsCfg<NX, NU, L, (int)sizeof(T), NI, FAM>;
     using REC = GpsRec<NX, NU, Cfg::SPW, (int)sizeof(T), FAM>;
-    GpsPlan p;
+    LaunchPlan p;
     const int SPW = Cfg::SPW;
     const tinympc_state_t &s = d.io.state;
-    // region B: previous box slacks (work->v / work->z) and family slacks, only when the caller wants them back
-    p.ly.has_b = (s.v || s.z || s.vcnew || s.zcnew || s.vlnew || s.zlnew || s.vlnew_tv || s.zlnew_tv) ? 1 : 0;
-    const int max_smem = d.max_smem_optin - 64;
     const size_t blob = ((size_t)(3 * NX * NX + 2 * NX * NU + NU * NU + 4 * NX + 2 * NU) * sizeof(T) + 15) / 16 * 16;
     using RINGH = GpsRing<NX, NU, L, (int)sizeof(T), NI, FAM>;
     const size_t per_warp = RINGH::WARP_BYTES, fixed = blob + RINGH::ZERO_BYTES;
-    if (fixed + per_warp > (size_t)max_smem) return p;
-    int maxw = (int)std::min<size_t>(gps_max_warps(NI), ((size_t)max_smem - fixed) / per_warp);
+    if (fixed + per_warp > (size_t)d.smem_budget) return p;
+    int maxw = (int)std::min<size_t>(gps_max_warps(NI), ((size_t)d.smem_budget - fixed) / per_warp);
     maxw = std::max(1, std::min(maxw, std::max(1, gps_env_int("TINYMPC_GPS_WARPS", gps_max_warps(NI)))));
     // balance the waves: with `waves` passes over the resident slots, use just enough warps per SM to hold B / waves
     const int64_t groups = (d.io.B + SPW - 1) / SPW;  // warps' worth of instances
     const int64_t cap = (int64_t)d.sm_count * maxw;
     const int64_t waves = std::max<int64_t>(1, (groups + cap - 1) / cap);
-    int warps = (int)std::min<int64_t>(maxw, std::max<int64_t>(1, (groups + waves * d.sm_count - 1) / (waves * d.sm_count)));
-    p.L = L;
-    p.NI = NI;
-    p.warps = warps;
+    const int warps = (int)std::min<int64_t>(maxw, std::max<int64_t>(1, (groups + waves * d.sm_count - 1) / (waves * d.sm_count)));
+    p.family = TINYMPC_KERNEL_GPS;
+    p.lanes = L;
+    p.group_instances = NI;
+    p.warps_resident = maxw;
+    p.instances_per_cta = warps * (32 / L) * NI;
+    p.threads = warps * 32;
     p.ctas = (int)std::max<int64_t>(1, std::min<int64_t>(d.sm_count, (groups + warps - 1) / warps));
     p.smem = fixed + per_warp * (size_t)warps;
-    p.ws_bytes = (size_t)p.ctas * warps * d.N * (REC::recA + (p.ly.has_b ? REC::recB : 0)) * sizeof(T);
+    // region B: previous box slacks (work->v / work->z) and family slacks, only when the caller wants them back
+    p.gps_has_b = (s.v || s.z || s.vcnew || s.zcnew || s.vlnew || s.zlnew || s.vlnew_tv || s.zlnew_tv) ? 1 : 0;
+    p.workspace_bytes = (size_t)p.ctas * warps * d.N * (REC::recA + (p.gps_has_b ? REC::recB : 0)) * sizeof(T);
     return p;
 }
 
 template <typename T, int NX, int NU, int L, int NI, int FAM, bool FAST>
-int launch_gps_cfg(LaunchDesc *d, const KParams<T, NX, NU> &P0) {
-    const GpsPlan plan = gps_plan_L<T, NX, NU, L, NI, FAM>(*d);
-    if (plan.L == 0 || !d->gmat || !d->work_queue) return TINYMPC_ERR_UNSUPPORTED;
-    d->out_ws_need = plan.ws_bytes;
-    if (!d->gps_ws || d->gps_ws_bytes < plan.ws_bytes) return TM_ERR_WORKSPACE;
+int launch_gps_cfg(LaunchDesc *d, const LaunchPlan &plan, const KParams<T, NX, NU> &P0) {
     KParams<T, NX, NU> P = P0;
-    P.gps = plan.ly;
-    P.gps_ws = (T *)d->gps_ws;
+    P.gps.has_b = plan.gps_has_b;
+    P.gps_ws = (T *)d->workspace;
     auto kern = gps_solve_kernel<T, NX, NU, L, NI, FAM, FAST>;
     if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)plan.smem) != cudaSuccess) return TINYMPC_ERR_CUDA;
-    kern<<<plan.ctas, plan.warps * 32, plan.smem, d->stream>>>(P, (const T *)d->gmat, (unsigned long long *)d->work_queue);
-    d->out_threads = plan.warps * 32;
-    d->out_ctas = plan.ctas;
-    d->out_smem = (int)plan.smem;
-    d->out_lanes_per_instance = L;
-    d->out_instances_per_cta = plan.warps * (32 / L) * NI;
-    d->out_tmem_cols = 0;
+    kern<<<plan.ctas, plan.threads, plan.smem, d->stream>>>(P, (const T *)d->gmat, (unsigned long long *)d->work_queue);
     return cudaGetLastError() == cudaSuccess ? TINYMPC_OK : TINYMPC_ERR_CUDA;
 }
 
@@ -1255,38 +1241,37 @@ inline int gps_family_mask(const LaunchDesc &d) {
     return !soc && !lin ? 0 : (soc && !lin ? 1 : (!soc ? 6 : 7));
 }
 
-template <typename T, int NX, int NU, bool FAST>
-int launch_gps(LaunchDesc *d, const KParams<T, NX, NU> &P0) {
+// The compiled variant that serves d, for the planner and the launcher alike: f(IdxTag<L>, IdxTag<NI>, IdxTag<FAM>) with
+// the shape's lane width L, the family mask FAM of d and NI instances per lane group; `none` when the shape has no
+// variant.  Only the planner's NI is compiled; -DTM_GPS_TUNE also builds the one-instance variant of the shapes that
+// default to two, which ni = 1 selects (developer sweeps).
+template <typename T, int NX, int NU, typename R, typename F>
+R gps_variant(const LaunchDesc &d, int ni, R none, F &&f) {
     constexpr int L = gps_pick_L<T, NX, NU>();
     if constexpr (L == 0) {
-        return TINYMPC_ERR_UNSUPPORTED;
+        return none;
     } else {
         constexpr int NIP = gps_pick_NI<T, NX, NU, L>();
-        const int fam = gps_family_mask(*d);
-        int ni = gps_env_int("TINYMPC_GPS_NI", NIP);
-        if (ni != 1 && ni != 2) ni = NIP;
-        if (ni > NIP) ni = NIP;
+        const int fam = gps_family_mask(d);
         (void)ni;
-// only the planner's instances-per-group variant is compiled; -DTM_GPS_TUNE also builds the one-instance variant of the
-// shapes that default to two (TINYMPC_GPS_NI=1 then selects it: developer sweeps)
 #ifdef TM_GPS_TUNE
-#define TM_GPS_CASE(FF)                                                                   \
-    if (fam == FF) {                                                                      \
-        if constexpr (NIP == 2) {                                                         \
-            if (ni == 2) return launch_gps_cfg<T, NX, NU, L, 2, FF, FAST>(d, P0);         \
-        }                                                                                 \
-        return launch_gps_cfg<T, NX, NU, L, 1, FF, FAST>(d, P0);                          \
+#define TM_GPS_CASE(FF)                                                  \
+    if (fam == FF) {                                                     \
+        if constexpr (NIP == 2) {                                        \
+            if (ni == 1) return f(IdxTag<L>{}, IdxTag<1>{}, IdxTag<FF>{}); \
+        }                                                                \
+        return f(IdxTag<L>{}, IdxTag<NIP>{}, IdxTag<FF>{});              \
     }
 #else
 #define TM_GPS_CASE(FF) \
-    if (fam == FF) return launch_gps_cfg<T, NX, NU, L, NIP, FF, FAST>(d, P0);
+    if (fam == FF) return f(IdxTag<L>{}, IdxTag<NIP>{}, IdxTag<FF>{});
 #endif
         TM_GPS_CASE(0)
         TM_GPS_CASE(1)
         TM_GPS_CASE(6)
         TM_GPS_CASE(7)
 #undef TM_GPS_CASE
-        return TINYMPC_ERR_UNSUPPORTED;
+        return none;
     }
 }
 

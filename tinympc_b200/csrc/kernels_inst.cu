@@ -20,11 +20,10 @@
 #define TM_SYM(prefix) TM_CAT(prefix, TM_NX, TM_NU)
 
 // cross-part entry points of this dimension pair
-extern "C" int TM_SYM(tm_gpi_launch_)(tmpc::LaunchDesc *d);
-extern "C" int TM_SYM(tm_gpi_fit_)(int dtype, int N, int max_smem_optin);
-extern "C" int TM_SYM(tm_gpi_ipc_)(int dtype, int N, int max_smem_optin);
-extern "C" int TM_SYM(tm_gps_launch_)(tmpc::LaunchDesc *d);
-extern "C" int TM_SYM(tm_gps_lanes_)(int dtype);
+extern "C" tmpc::LaunchPlan TM_SYM(tm_gpi_plan_)(const tmpc::LaunchDesc &d);
+extern "C" int TM_SYM(tm_gpi_launch_)(tmpc::LaunchDesc *d, const tmpc::LaunchPlan &plan);
+extern "C" tmpc::LaunchPlan TM_SYM(tm_gps_plan_)(const tmpc::LaunchDesc &d);
+extern "C" int TM_SYM(tm_gps_launch_)(tmpc::LaunchDesc *d, const tmpc::LaunchPlan &plan);
 
 #if TM_PART == 0
 // =========================================================================================================
@@ -34,35 +33,71 @@ extern "C" int TM_SYM(tm_gps_lanes_)(int dtype);
 namespace tmpc {
 namespace {
 
+// bytes of one [N][vectors][Bpad] state / input array of the structure-of-arrays workspace
+template <typename T>
+size_t tpi_szx(const LaunchDesc &d) { return (size_t)d.N * SoA<T, TM_NX>::NV * 16 * d.Bpad; }
+template <typename T>
+size_t tpi_szu(const LaunchDesc &d) { return (size_t)(d.N - 1) * SoA<T, TM_NU>::NV * 16 * d.Bpad; }
+
+template <typename T>
+LaunchPlan tpi_plan(const LaunchDesc &d) {
+    LaunchPlan p;
+    if (d.io.models) return p;  // per-instance models live in the on-chip kernel's per-lane registers only
+    p.family = TINYMPC_KERNEL_TPI;
+    p.lanes = 1;
+    p.threads = p.instances_per_cta = TPI_THREADS;
+    p.ctas = (int)((d.io.B + TPI_THREADS - 1) / TPI_THREADS);
+    // vnew (two buffers), g, znew (two buffers), y, d, and a slack / dual pair per enabled constraint family; 256 bytes slack
+    const size_t nx_arrays = 3 + 2 * (d.soc_x + d.lin_x + d.tvl_x), nu_arrays = 4 + 2 * (d.soc_u + d.lin_u + d.tvl_u);
+    p.workspace_bytes = nx_arrays * tpi_szx<T>(d) + nu_arrays * tpi_szu<T>(d) + 256;
+    return p;
+}
+
 template <typename T, bool FAST, bool EXT>
-int launch_tpi(LaunchDesc *d) {
+int launch_tpi(LaunchDesc *d, const LaunchPlan &plan) {
     KParams<T, TM_NX, TM_NU> P;
     fill_params<T, TM_NX, TM_NU>(P, *d);
-    const int threads = TPI_THREADS;
-    const int64_t blocks = (d->io.B + threads - 1) / threads;
-    if (blocks <= 0) return TINYMPC_OK;
-    tpi_solve_kernel<T, TM_NX, TM_NU, FAST, EXT><<<(unsigned)blocks, threads, 0, d->stream>>>(P);
-    d->out_threads = threads;
-    d->out_ctas = (int)blocks;
-    d->out_smem = 0;
-    d->out_lanes_per_instance = 1;
-    d->out_instances_per_cta = threads;
-    d->out_tmem_cols = 0;
+    // carve the workspace in tpi_plan's order (the arrays of disabled families stay null)
+    const size_t szx = tpi_szx<T>(*d), szu = tpi_szu<T>(*d);
+    char *c = (char *)d->workspace;
+    auto take = [&](size_t n) {
+        void *r = c;
+        c += n;
+        return r;
+    };
+    P.w_v[0] = take(szx); P.w_v[1] = take(szx); P.w_g = take(szx);
+    P.w_z[0] = take(szu); P.w_z[1] = take(szu); P.w_y = take(szu); P.w_d = take(szu);
+    if (d->soc_x) { P.w_vc = take(szx); P.w_gc = take(szx); }
+    if (d->soc_u) { P.w_zc = take(szu); P.w_yc = take(szu); }
+    if (d->lin_x) { P.w_vl = take(szx); P.w_gl = take(szx); }
+    if (d->lin_u) { P.w_zl = take(szu); P.w_yl = take(szu); }
+    if (d->tvl_x) { P.w_vlt = take(szx); P.w_glt = take(szx); }
+    if (d->tvl_u) { P.w_zlt = take(szu); P.w_ylt = take(szu); }
+    tpi_solve_kernel<T, TM_NX, TM_NU, FAST, EXT><<<(unsigned)plan.ctas, plan.threads, 0, d->stream>>>(P);
     return cudaGetLastError() == cudaSuccess ? TINYMPC_OK : TINYMPC_ERR_CUDA;
 }
 
 template <typename T>
-int launch_T(LaunchDesc *d) {
-    if (d->io.models) return TINYMPC_ERR_UNSUPPORTED;  // per-instance models live in the on-chip kernel's per-lane registers only
-    if (d->ext) return d->fast ? launch_tpi<T, true, true>(d) : launch_tpi<T, false, true>(d);
-    return d->fast ? launch_tpi<T, true, false>(d) : launch_tpi<T, false, false>(d);
+int launch_T(LaunchDesc *d, const LaunchPlan &plan) {
+    if (d->ext) return d->fast ? launch_tpi<T, true, true>(d, plan) : launch_tpi<T, false, true>(d, plan);
+    return d->fast ? launch_tpi<T, true, false>(d, plan) : launch_tpi<T, false, false>(d, plan);
 }
 
-int launch(LaunchDesc *d) {
-    if (d->family == TINYMPC_KERNEL_GPI) return TM_SYM(tm_gpi_launch_)(d);
-    if (d->family == TINYMPC_KERNEL_GPS) return TM_SYM(tm_gps_launch_)(d);
-    if (d->dtype == TINYMPC_F32) return launch_T<float>(d);
-    if (d->dtype == TINYMPC_F64) return launch_T<double>(d);
+LaunchPlan plan(const LaunchDesc &d, int family) {
+    if (family == TINYMPC_KERNEL_GPI) return TM_SYM(tm_gpi_plan_)(d);
+    if (family == TINYMPC_KERNEL_GPS) return TM_SYM(tm_gps_plan_)(d);
+    if (family != TINYMPC_KERNEL_TPI) return {};
+    if (d.dtype == TINYMPC_F32) return tpi_plan<float>(d);
+    if (d.dtype == TINYMPC_F64) return tpi_plan<double>(d);
+    return {};
+}
+
+int launch(LaunchDesc *d, const LaunchPlan &plan) {
+    if (plan.family == TINYMPC_KERNEL_GPI) return TM_SYM(tm_gpi_launch_)(d, plan);
+    if (plan.family == TINYMPC_KERNEL_GPS) return TM_SYM(tm_gps_launch_)(d, plan);
+    if (plan.family != TINYMPC_KERNEL_TPI) return TINYMPC_ERR_UNSUPPORTED;
+    if (d->dtype == TINYMPC_F32) return launch_T<float>(d, plan);
+    if (d->dtype == TINYMPC_F64) return launch_T<double>(d, plan);
     return TINYMPC_ERR_ARG;
 }
 
@@ -79,13 +114,7 @@ int precompute_batch(int dtype, int64_t B, const void *A, const void *Bm, const 
 }  // namespace tmpc
 
 extern "C" const tmpc::DimEntry *TM_SYM(tm_dim_entry_)() {
-    static const tmpc::DimEntry e = {TM_NX,
-                                     TM_NU,
-                                     &tmpc::launch,
-                                     &TM_SYM(tm_gpi_fit_),
-                                     &TM_SYM(tm_gpi_ipc_),
-                                     &tmpc::precompute_batch,
-                                     &TM_SYM(tm_gps_lanes_)};
+    static const tmpc::DimEntry e = {TM_NX, TM_NU, &tmpc::plan, &tmpc::launch, &tmpc::precompute_batch};
     return &e;
 }
 
@@ -98,16 +127,15 @@ namespace tmpc {
 namespace {
 
 template <typename T, int NX, int NU, bool FAST>
-int launch_gpi(LaunchDesc *d) {
-    const GpiPlan plan = gpi_plan<T, NX, NU>(d->N, d->max_smem_optin - 64);
-    if (plan.L == 0 || !d->gmat || !d->work_queue) return TINYMPC_ERR_UNSUPPORTED;
+int launch_gpi(LaunchDesc *d, const LaunchPlan &plan) {
     KParams<T, NX, NU> P;
     fill_params<T, NX, NU>(P, *d);
     const T *gmat = (const T *)d->gmat;
     const bool het = d->io.models != nullptr;  // heterogeneous batch: per-instance model blobs
+    const bool tm = plan.tmem_cols != 0;
     // STRICT, shared model, tensor-memory plan (the headline path): min / max clamp when no bound is a signed zero
 #define TM_GPI_CASE(LL, HH, TT)                                                                                          \
-    if (plan.L == LL && het == HH && plan.tm == TT) {                                                                    \
+    if (plan.lanes == LL && het == HH && tm == TT) {                                                                     \
         if constexpr (!FAST && !HH && TT && sizeof(T) == 4) {                                                            \
             if (d->bounds_zero_free) return launch_gpi_L<T, NX, NU, LL, FAST, HH, TT, true>(d, plan, P, gmat);           \
         }                                                                                                                \
@@ -128,35 +156,19 @@ int launch_gpi(LaunchDesc *d) {
     return TINYMPC_ERR_UNSUPPORTED;
 }
 
-template <typename T>
-int launch_T(LaunchDesc *d) {
-    if (d->ext) return TINYMPC_ERR_UNSUPPORTED;  // the on-chip kernel covers box constraints; the rest streams (gps)
-    return d->fast ? launch_gpi<T, TM_NX, TM_NU, true>(d) : launch_gpi<T, TM_NX, TM_NU, false>(d);
-}
-
 }  // namespace
 }  // namespace tmpc
 
-extern "C" int TM_SYM(tm_gpi_launch_)(tmpc::LaunchDesc *d) {
-    if (d->dtype == TINYMPC_F32) return tmpc::launch_T<float>(d);
-    if (d->dtype == TINYMPC_F64) return tmpc::launch_T<double>(d);
+extern "C" tmpc::LaunchPlan TM_SYM(tm_gpi_plan_)(const tmpc::LaunchDesc &d) {
+    if (d.ext) return {};  // the on-chip kernel covers box constraints; the rest streams (gps)
+    if (d.dtype == TINYMPC_F32) return tmpc::gpi_plan<float, TM_NX, TM_NU>(d);
+    if (d.dtype == TINYMPC_F64) return tmpc::gpi_plan<double, TM_NX, TM_NU>(d);
+    return {};
+}
+extern "C" int TM_SYM(tm_gpi_launch_)(tmpc::LaunchDesc *d, const tmpc::LaunchPlan &plan) {
+    if (d->dtype == TINYMPC_F32) return d->fast ? tmpc::launch_gpi<float, TM_NX, TM_NU, true>(d, plan) : tmpc::launch_gpi<float, TM_NX, TM_NU, false>(d, plan);
+    if (d->dtype == TINYMPC_F64) return d->fast ? tmpc::launch_gpi<double, TM_NX, TM_NU, true>(d, plan) : tmpc::launch_gpi<double, TM_NX, TM_NU, false>(d, plan);
     return TINYMPC_ERR_ARG;
-}
-extern "C" int TM_SYM(tm_gpi_fit_)(int dtype, int N, int max_smem_optin) {
-    if (dtype == TINYMPC_F32) return tmpc::gpi_fit_T<float, TM_NX, TM_NU>(N, max_smem_optin - 64);
-    if (dtype == TINYMPC_F64) return tmpc::gpi_fit_T<double, TM_NX, TM_NU>(N, max_smem_optin - 64);
-    return 0;
-}
-extern "C" int TM_SYM(tm_gpi_ipc_)(int dtype, int N, int max_smem_optin) {
-    if (dtype == TINYMPC_F32) {
-        const tmpc::GpiPlan p = tmpc::gpi_plan<float, TM_NX, TM_NU>(N, max_smem_optin - 64);
-        return p.L ? ((p.warps << 16) | (p.warps * (32 / p.L))) : 0;
-    }
-    if (dtype == TINYMPC_F64) {
-        const tmpc::GpiPlan p = tmpc::gpi_plan<double, TM_NX, TM_NU>(N, max_smem_optin - 64);
-        return p.L ? ((p.warps << 16) | (p.warps * (32 / p.L))) : 0;
-    }
-    return 0;
 }
 
 #else
@@ -167,34 +179,34 @@ namespace tmpc {
 namespace {
 
 template <typename T>
-int launch_T(LaunchDesc *d) {
-    if (d->io.models) return TINYMPC_ERR_UNSUPPORTED;
+LaunchPlan plan_T(const LaunchDesc &d) {
+    if (d.io.models) return {};  // per-instance models live in the on-chip kernel only
+    return gps_variant<T, TM_NX, TM_NU>(d, gps_env_int("TINYMPC_GPS_NI", 0), LaunchPlan{}, [&](auto l, auto ni, auto fam) {
+        return gps_plan_L<T, TM_NX, TM_NU, decltype(l)::value, decltype(ni)::value, decltype(fam)::value>(d);
+    });
+}
+
+template <typename T>
+int launch_T(LaunchDesc *d, const LaunchPlan &plan) {
     KParams<T, TM_NX, TM_NU> P;
     fill_params<T, TM_NX, TM_NU>(P, *d);
-    return d->fast ? launch_gps<T, TM_NX, TM_NU, true>(d, P) : launch_gps<T, TM_NX, TM_NU, false>(d, P);
+    return gps_variant<T, TM_NX, TM_NU>(*d, plan.group_instances, (int)TINYMPC_ERR_UNSUPPORTED, [&](auto l, auto ni, auto fam) {
+        constexpr int L = decltype(l)::value, NI = decltype(ni)::value, FAM = decltype(fam)::value;
+        return d->fast ? launch_gps_cfg<T, TM_NX, TM_NU, L, NI, FAM, true>(d, plan, P) : launch_gps_cfg<T, TM_NX, TM_NU, L, NI, FAM, false>(d, plan, P);
+    });
 }
 
 }  // namespace
 }  // namespace tmpc
 
-extern "C" int TM_SYM(tm_gps_launch_)(tmpc::LaunchDesc *d) {
-    if (d->dtype == TINYMPC_F32) return tmpc::launch_T<float>(d);
-    if (d->dtype == TINYMPC_F64) return tmpc::launch_T<double>(d);
-    return TINYMPC_ERR_ARG;
+extern "C" tmpc::LaunchPlan TM_SYM(tm_gps_plan_)(const tmpc::LaunchDesc &d) {
+    if (d.dtype == TINYMPC_F32) return tmpc::plan_T<float>(d);
+    if (d.dtype == TINYMPC_F64) return tmpc::plan_T<double>(d);
+    return {};
 }
-// lanes per instance of the streamed lane-group kernel for this shape (0 = not available)
-extern "C" int TM_SYM(tm_gps_lanes_)(int dtype) {
-    // lanes per instance in bits 0-7, instances per lane group (1 or 2) in bits 8-15
-    if (dtype == TINYMPC_F32) {
-        constexpr int Lf = tmpc::gps_pick_L<float, TM_NX, TM_NU>();
-        if constexpr (Lf == 0) return 0;
-        else return Lf | (tmpc::gps_pick_NI<float, TM_NX, TM_NU, Lf>() << 8);
-    }
-    if (dtype == TINYMPC_F64) {
-        constexpr int Ld = tmpc::gps_pick_L<double, TM_NX, TM_NU>();
-        if constexpr (Ld == 0) return 0;
-        else return Ld | (tmpc::gps_pick_NI<double, TM_NX, TM_NU, Ld>() << 8);
-    }
-    return 0;
+extern "C" int TM_SYM(tm_gps_launch_)(tmpc::LaunchDesc *d, const tmpc::LaunchPlan &plan) {
+    if (d->dtype == TINYMPC_F32) return tmpc::launch_T<float>(d, plan);
+    if (d->dtype == TINYMPC_F64) return tmpc::launch_T<double>(d, plan);
+    return TINYMPC_ERR_ARG;
 }
 #endif

@@ -73,12 +73,7 @@ inline void fill_params(KParams<T, NX, NU> &P, const LaunchDesc &d) {
     P.iter = io.iter; P.solved = io.solved; P.residuals = (T *)io.residuals;
     P.u0 = (T *)io.u0;
     P.models = (const T *)io.models;
-    P.gpi_vscratch = (T *)d.gpi_vscratch;
-    P.w_v[0] = d.w_v[0]; P.w_v[1] = d.w_v[1]; P.w_z[0] = d.w_z[0]; P.w_z[1] = d.w_z[1];
-    P.w_g = d.w_g; P.w_y = d.w_y; P.w_d = d.w_d;
-    P.w_vc = d.w_vc; P.w_zc = d.w_zc; P.w_gc = d.w_gc; P.w_yc = d.w_yc;
-    P.w_vl = d.w_vl; P.w_zl = d.w_zl; P.w_gl = d.w_gl; P.w_yl = d.w_yl;
-    P.w_vlt = d.w_vlt; P.w_zlt = d.w_zlt; P.w_glt = d.w_glt; P.w_ylt = d.w_ylt;
+    P.gpi_vscratch = (T *)d.scratch;
 }
 
 }  // namespace tmpc

@@ -11,7 +11,6 @@ namespace tmpc {
 struct LaunchDesc {
     int dtype;   // TINYMPC_F32 / F64
     int fast;    // TINYMPC_MODE_FAST ?
-    int family;  // TINYMPC_KERNEL_TPI / GPI / GPS (resolved, never AUTO)
     int ext;     // any of soc / linear / tv-linear enabled
 
     // host copies of the model + cache in the native dtype (column-major)
@@ -30,44 +29,44 @@ struct LaunchDesc {
     const void *Alin_x, *blin_x, *Alin_u, *blin_u, *tv_Alin_x, *tv_blin_x, *tv_Alin_u, *tv_blin_u;
     tinympc_batch_t io;  // device pointers
     int64_t Bpad;
-    void *w_v[2], *w_z[2], *w_g, *w_y, *w_d;
-    void *w_vc, *w_zc, *w_gc, *w_yc, *w_vl, *w_zl, *w_gl, *w_yl, *w_vlt, *w_zlt, *w_glt, *w_ylt;
     const void *gmat;  // device blob: A,B,f,Qd,Rd,Kinf,Pinf,Quu,AmBKt,APf,BPf packed (native dtype)
     int bounds_tv;
     int bounds_zero_free;  // no element of the box bounds is +-0 (lets STRICT kernels clamp with min / max instructions)
     const void *h_xlo, *h_xhi, *h_ulo, *h_uhi;  // host copies of column 0 of the bounds (native dtype), may be null
-    void *work_queue;  // GPI: device int64 counter (zeroed by the caller)
-    void *gpi_vscratch;  // GPI: scratch for work->v / work->z persistence (allocated by the caller when state.v/z given)
-    void *gps_ws;        // GPS: streamed state records of the resident slots (allocated by the caller, see out_ws_need)
-    size_t gps_ws_bytes;
+    void *work_queue;  // GPI / GPS: device int64 counter (zeroed by the caller)
+    void *workspace;   // TPI / GPS: LaunchPlan::workspace_bytes, allocated by the caller
+    void *scratch;     // GPI: LaunchPlan::scratch_bytes, allocated by the caller (null when the plan needs none)
 
     cudaStream_t stream;
     int sm_count;
-    int max_smem_optin;
-
-    // filled by the launcher
-    int out_threads, out_ctas, out_smem, out_lanes_per_instance, out_instances_per_cta, out_tmem_cols;
-    size_t out_ws_need;  // GPS: workspace bytes this launch needs (set when the launcher returns TM_ERR_WORKSPACE)
+    int smem_budget;  // dynamic shared memory a CTA may use: the opt-in limit less 64 bytes of static shared memory
 };
 
-// internal: the launcher needs a larger gps_ws (size in out_ws_need); never leaves the library
-constexpr int TM_ERR_WORKSPACE = -100;
+// How one solve runs, decided by the kernel family's own translation unit before anything is allocated or launched:
+// the caller allocates from it, launches with it and reports it through tinympc_b200_stats_t.
+struct LaunchPlan {
+    int family = 0;              // TINYMPC_KERNEL_TPI / GPI / GPS; 0 = this family cannot serve the solve
+    int lanes = 0;               // lanes per instance (TPI: 1)
+    int group_instances = 0;     // GPS: instances per lane group
+    int tmem_cols = 0;           // GPI: tensor-memory columns per CTA (0 = the whole state in shared memory)
+    int warps_resident = 0;      // GPI / GPS: warps per CTA the on-chip memory holds
+    int instances_per_cta = 0;   // GPI: capacity (warps_resident); GPS: of this launch; TPI: threads per CTA
+    int ctas = 0, threads = 0;   // launch geometry for this batch
+    size_t smem = 0;             // dynamic shared memory per CTA
+    size_t workspace_bytes = 0;  // TPI structure-of-arrays / GPS state records
+    size_t scratch_bytes = 0;    // GPI: previous-slack scratch, when state.v / state.z is requested
+    int gps_has_b = 0;           // GPS: the records carry region B (previous / family slacks)
+};
 
-// per-(nx,nu) entry: returns 0 on success, TINYMPC_ERR_UNSUPPORTED when (dtype,family,...) is not compiled
-typedef int (*launch_fn)(LaunchDesc *);
-
+// per-(nx,nu) entry.  plan: host arithmetic only, no CUDA calls.  launch: 0 on success, TINYMPC_ERR_UNSUPPORTED when
+// the planned variant is not compiled, TINYMPC_ERR_CUDA when the launch fails.
 struct DimEntry {
     int nx, nu;
-    launch_fn launch;
-    // GPI capability query: shared-memory bytes per CTA for a given (dtype, N) or 0 if GPI not available
-    int (*gpi_fit)(int dtype, int N, int max_smem_optin);
-    // GPI plan for (dtype, N): (warps per CTA << 16) | instances resident per CTA; 0 if GPI is not available
-    int (*gpi_instances_per_cta)(int dtype, int N, int max_smem_optin);
+    LaunchPlan (*plan)(const LaunchDesc &d, int family);
+    int (*launch)(LaunchDesc *d, const LaunchPlan &plan);
     // batched cache precompute on the device (precompute_kernel.cuh): device pointers, one model blob per instance
     int (*precompute_batch)(int dtype, int64_t B, const void *A, const void *Bm, const void *f, const void *Qdiag, const void *Rdiag,
                             const void *rho, void *models_out, int32_t *sweeps_out, int sm_count, cudaStream_t stream);
-    // streamed lane-group kernel (gps_kernel.cuh): lanes per instance (bits 0-7) | instances per lane group << 8; 0 = shape not available
-    int (*gps_lanes)(int dtype);
 };
 
 }  // namespace tmpc
