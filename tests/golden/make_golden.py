@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Generate the golden fixtures from the UNMODIFIED reference (run in the build container only).
 
-    python tests/golden/make_golden.py [closed_loop] [reference]
+    python tests/golden/make_golden.py [closed_loop] [reference] [families]
 
 closed_loop — for each parity case (tests/helpers.py:make_cases) this runs the reference — compiled with the pinned flags
 into oracle/_ref/libtinympc_ref_{f64,f32}.so by oracle/Makefile — through a warm-started closed loop and stores,
@@ -17,6 +17,10 @@ reference — tests/golden/reference/: the reference's outputs for the other tes
   * tiny_setup_<dtype>.npz  the cache tiny_setup computes for tests/helpers.py:precompute_models,
   * sensitivity_tables.npz  the tables tiny_initialize_sensitivity_matrices leaves,
   * examples/<name>.txt.gz  what the reference's example programs print (oracle/_ref/examples_ref, oracle/Makefile).
+
+families — tests/golden/reference/families_<dtype>.npz: the cones / hyperplanes cases (tests/helpers.py:family_cases), in the
+lti_sweep format: per case the cache tiny_setup computed, the x0 of every step, and the digests of every output and every one
+of the 20 state arrays of a warm-started three-step loop.  Written on its own so that the other fixtures stay untouched.
 """
 import ctypes as C
 import gzip
@@ -79,6 +83,19 @@ def reference_outputs():
         print(f"examples/{name}.txt.gz: {os.path.getsize(path)} bytes")
 
 
+def family_outputs():
+    for dt in (np.float32, np.float64):
+        out, digests = {}, {}
+        for key, sp, inst in H.family_cases(dt):
+            prob = H.problem_from_spec(sp, dt, oracle.ref_setup)
+            res, x0s = H.closed_loop(prob, sp.settings, inst, 3, False, H.ALL_STATE, _reference)
+            out.update({f"{key}_{f}": getattr(prob, f) for f in H.CACHE_FIELDS})
+            out[f"{key}_x0_seq"] = np.stack(x0s)
+            for k, r in enumerate(res):
+                digests.update({f"{key}_step{k}_{n}": H.digest(r[n]) for n in H.OUT_KEYS + H.ALL_STATE})
+        _save(f"families_{np.dtype(dt).name}", dict(out, names=np.array(list(digests)), digests=np.array(list(digests.values()))))
+
+
 def closed_loop_fixtures():
     cases = H.make_cases()
     for name in sorted(cases):
@@ -112,5 +129,5 @@ def closed_loop_fixtures():
 
 
 if __name__ == "__main__":
-    for part in sys.argv[1:] or ["closed_loop", "reference"]:
-        {"closed_loop": closed_loop_fixtures, "reference": reference_outputs}[part]()
+    for part in sys.argv[1:] or ["closed_loop", "reference", "families"]:
+        {"closed_loop": closed_loop_fixtures, "reference": reference_outputs, "families": family_outputs}[part]()

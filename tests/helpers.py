@@ -74,6 +74,81 @@ def lti_sweep(dt):
     return out
 
 
+# Shapes of the constraint-family cases and the streamed lane-group variant (lanes per instance L, instances per warp =
+# 32 / L x instances per lane group) each one runs on, per dtype (gps_pick_L / gps_pick_NI in csrc/gps_kernel.cuh)
+FAMILY_VARIANTS = {
+    np.float32: {(6, 3): (4, 16), (4, 8): (4, 16), (8, 8): (4, 16), (12, 4): (4, 16), (12, 8): (4, 8), (16, 8): (8, 4)},
+    np.float64: {(6, 3): (4, 16), (4, 8): (4, 8), (8, 8): (8, 8), (12, 4): (8, 4), (12, 8): (16, 2), (16, 8): (16, 2)},
+}
+# constraint mixes: which settings flags each one enables on top of the box bounds
+FAMILY_MIXES = {
+    "C": ("en_state_soc", "en_input_soc"),
+    "H": ("en_state_linear", "en_input_linear", "en_tv_state_linear", "en_tv_input_linear"),
+    "CH": ("en_state_soc", "en_input_soc", "en_state_linear", "en_input_linear"),
+    "ALL": ("en_state_soc", "en_input_soc", "en_state_linear", "en_input_linear", "en_tv_state_linear", "en_tv_input_linear"),
+}
+FAMILY_FLAGS = ("en_state_bound", "en_input_bound") + FAMILY_MIXES["ALL"]
+# cone start rows per state / input dimension: 2-4 state cones and 1-2 input cones, the last of each ending on the last row
+# (where the padding lanes of the wider lane groups begin); every cone satisfies start + 3 <= n
+STATE_CONES = {4: [0, 1], 6: [0, 3], 8: [0, 2, 5], 12: [0, 4, 7, 9], 16: [1, 6, 10, 13]}
+INPUT_CONES = {3: [0], 4: [0, 1], 8: [2, 5]}
+
+
+def family_spec(nx, nu, mix, N=12, seed=0) -> wl.ModelSpec:
+    """A random LTI problem with active box bounds and the constraint families of `mix` (FAMILY_MIXES): second-order cones
+    on the state and the input, static hyperplanes (two state rows, one input row), time-varying hyperplanes (one row per
+    knot point and side)."""
+    sp = wl.random_lti(nx, nu, N, seed=seed)
+    rng = np.random.default_rng(500 + 31 * nx + nu + seed)
+    cx, cu = STATE_CONES[nx], INPUT_CONES[nu]
+    assert all(0 <= c and c + 3 <= nx for c in cx) and all(0 <= c and c + 3 <= nu for c in cu)
+    cons = dict(x_min=np.full(nx, -3.0), x_max=np.full(nx, 3.0), u_min=np.full(nu, -0.8), u_max=np.full(nu, 0.8))
+    flags = FAMILY_MIXES[mix]
+    if "en_state_soc" in flags:
+        cons.update(Acx=cx, qcx=[3] * len(cx), cx=rng.uniform(0.5, 1.5, len(cx)).tolist(),
+                    Acu=cu, qcu=[3] * len(cu), cu=rng.uniform(0.5, 1.0, len(cu)).tolist())
+    if "en_state_linear" in flags:
+        cons.update(Alin_x=rng.standard_normal((2, nx)) / np.sqrt(nx), blin_x=rng.uniform(1.0, 2.0, 2),
+                    Alin_u=rng.standard_normal((1, nu)) / np.sqrt(nu), blin_u=rng.uniform(0.3, 0.6, 1))
+    if "en_tv_state_linear" in flags:
+        cons.update(tv_Alin_x=rng.standard_normal((N, nx)) / np.sqrt(nx), tv_blin_x=rng.uniform(1.0, 2.0, (1, N)),
+                    tv_Alin_u=rng.standard_normal((N - 1, nu)) / np.sqrt(nu), tv_blin_u=rng.uniform(0.3, 0.6, (1, N - 1)))
+    sp.constraints = cons
+    s = copy_settings(sp.settings)
+    for f in flags:
+        setattr(s, f, 1)
+    s.max_iter = 80
+    s.abs_pri_tol = s.abs_dua_tol = 1e-2
+    sp.settings = s
+    return sp
+
+
+def family_x0(spec, rng, B):
+    """Initial states for family_spec problems: the even instances start small and deep inside every state cone (they can
+    converge), the odd ones at a random point up to three times further out (they typically run to max_iter)."""
+    x0 = rng.standard_normal((B, spec.nx)) * np.where(np.arange(B) % 2 == 0, 0.1, rng.uniform(1.0, 3.5, B))[:, None]
+    if spec.settings.en_state_soc:
+        for s, mu in zip(spec.constraints.get("Acx", []), spec.constraints.get("cx", [])):
+            inside = np.abs(x0[:, s + 2]) + 1.5 * np.linalg.norm(x0[:, s:s + 2], axis=1) / mu + 0.3
+            x0[::2, s + 2] = inside[::2]
+    return x0
+
+
+def family_cases(dt):
+    """Every shape of FAMILY_VARIANTS x every mix of FAMILY_MIXES -> [(key, spec, inst)]: N = 12, 7 instances (an odd count,
+    so the last lane group of a two-instance group is half padding), check_termination 1 or 2, x0 spread so that some
+    instances converge before max_iter and some do not; run as warm-started three-step loops carrying every state array."""
+    out = []
+    for n, (nx, nu) in enumerate(FAMILY_VARIANTS[dt]):
+        for m, mix in enumerate(FAMILY_MIXES):
+            sp = family_spec(nx, nu, mix, seed=60 + n)
+            sp.settings.check_termination = 1 + (n + m) % 2
+            inst = wl.random_instances(7, nx, sp.N, seed=90 + 4 * n + m, dtype=dt)
+            inst["x0"] = family_x0(sp, np.random.default_rng(90 + 4 * n + m), 7).astype(dt)
+            out.append((f"{nx}_{nu}_{mix}", sp, inst))
+    return out
+
+
 def precompute_models():
     """[(nx, nu, [spec])]: the models whose tiny_setup cache the device precompute is checked against."""
     return [(12, 4, [wl.quadrotor(N=10), wl.quadrotor(N=10, hz=50)] + [wl.random_lti(12, 4, 10, seed=i) for i in range(6)]),

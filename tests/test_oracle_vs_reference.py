@@ -58,3 +58,34 @@ def test_port_bit_identical_to_reference_random_lti_sweep(dt):
         for k, p in enumerate(port):
             for name in H.OUT_KEYS + H.BOX_STATE:
                 assert H.digest(p[name]) == want[f"{key}_step{k}_{name}"], f"{key} step {k}: {name} differs"
+
+
+@pytest.mark.parametrize("dt", [np.float32, np.float64])
+def test_port_bit_identical_to_reference_constraint_families(dt):
+    """Cones and hyperplanes, alone and combined with active box bounds, on every shape of tests/helpers.py:family_cases:
+    warm-started three-step loops carrying all 20 state arrays, restatement vs the unmodified reference, bit for bit.  Every
+    enabled constraint family must change the answer, and the cases together must hold instances that converge before
+    max_iter and instances that run to it."""
+    from tinympc_b200.problem import copy_settings
+
+    gold = H.load_reference(f"families_{np.dtype(dt).name}")
+    want = dict(zip(gold["names"], gold["digests"]))
+    iters, max_iters = [], []
+    for key, sp, inst in H.family_cases(dt):
+        prob = H.problem_from_spec(sp, dt, H.stored_setup(gold, key))
+        port, x0s = H.closed_loop(prob, sp.settings, inst, 3, False, H.ALL_STATE, _solve("port"))
+        assert H.bits_equal(np.stack(x0s), gold[f"{key}_x0_seq"]), key
+        for k, p in enumerate(port):
+            for name in H.OUT_KEYS + H.ALL_STATE:
+                assert H.digest(p[name]) == want[f"{key}_step{k}_{name}"], f"{key} step {k}: {name} differs"
+            iters.append(p["iter"])
+            max_iters.append(np.full_like(p["iter"], sp.settings.max_iter))
+        for flag in H.FAMILY_FLAGS:
+            if getattr(sp.settings, flag):
+                off = copy_settings(sp.settings)
+                setattr(off, flag, 0)
+                o = _solve("port")(prob, off, inst["x0"], inst["Xref"], None, None, True, ())
+                assert not (H.bits_equal(o["sol_x"], port[0]["sol_x"]) and H.bits_equal(o["sol_u"], port[0]["sol_u"])), \
+                    f"{key}: {flag} does not change the solution"
+    iters, max_iters = np.concatenate(iters), np.concatenate(max_iters)
+    assert (iters < max_iters).any() and (iters == max_iters).any()
